@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA kernels)
     python bench.py --impl reference --gpus N --steps K ...   # CPU arm: the oracle port on host cores
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's results as DIR/*.npy
 
 Workload (BASELINE.json configs[1]): ``maximum_consecutive_dry_days`` (+ fused MissingAny valid
 count) on ONE synthetic daily float32 ``pr`` grid of shape (10950, 721, 1440) in mm/d, yearly
@@ -36,6 +37,7 @@ T_FULL, Y_FULL, X_FULL, YEAR = 10950, 721, 1440, 365
 METRIC = "grid_cells_per_s:maximum_consecutive_dry_days(10950x721x1440,f32)"
 UNIT = "grid-cells/s"
 ALL_SECTIONS = ("parity", "weak", "gather", "tx90p", "bootstrap", "eqm", "batch50", "e2e", "fwi", "cpu")
+DUMP_CELLS = 1 << 17   # --dump-outputs: 30 periods x 131,072 cells x 4 B x 2 arrays = 31 MB
 
 
 def parse_args():
@@ -51,7 +53,14 @@ def parse_args():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-tx90p", action="store_true")
     ap.add_argument("--cpu-lat", type=int, default=6, help="lat rows per worker of the bounded CPU sample")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (float32, (periods, cells), on a "
+                         f"fixed seeded sample of at most {DUMP_CELLS} cells of the grid)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     sec = [s for s in a.sections.split(",") if s]
     if a.no_e2e and "e2e" in sec:
         sec.remove("e2e")
@@ -210,6 +219,26 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------------ our arm
+def dump_outputs(path, out, valid, cell0, cells_total, rank, world):
+    """Writes what one step returns, (out, valid) of the (periods, cells) tile starting at global cell `cell0`, on
+    a sample of cells of the global grid that depends on nothing but its size: ``maximum_consecutive_dry_days.npy``
+    and ``valid_days.npy`` (days with data per period; MissingAny masks the periods short of 365), float32, cells
+    in global order."""
+    import torch
+    import torch.distributed as dist
+    sel = np.sort(np.random.default_rng(0).choice(cells_total, min(DUMP_CELLS, cells_total), replace=False))
+    mine = torch.from_numpy(sel[(sel >= cell0) & (sel < cell0 + out.shape[1])] - cell0).to(out.device)
+    parts = [(out[:, mine].cpu().numpy(), valid[:, mine].cpu().numpy().astype(np.float32))]
+    if world > 1:
+        gathered = [None] * world
+        dist.all_gather_object(gathered, parts[0])
+        parts = gathered
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+        for i, name in enumerate(("maximum_consecutive_dry_days", "valid_days")):
+            np.save(os.path.join(path, name + ".npy"), np.concatenate([p[i] for p in parts], axis=1))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -286,6 +315,8 @@ def run_ours(args):
     out_max = float(out.max().item())
     n_missing = int((valid != YEAR).sum().item())
     assert 0 <= out_max <= YEAR
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, valid, r0 * X, Yg * X, rank, world)
 
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,

@@ -100,9 +100,13 @@ def ffmc_step(t, p, w, h, f0):
 
 def dmc_step(t, p, h, mth, lat_band, d0):
     """Duff moisture code after one day (322-393).  ``lat_band`` = :func:`day_length_band` of the cells.
-    ``np.log(dmc0)`` is a float32 operation under numba (float32 argument), everything else float64."""
+    ``np.log(dmc0)`` is a float32 operation under numba (float32 argument), everything else float64.  numba calls
+    the C library's ``logf``, which rounds (all but) correctly.  numpy's own SIMD float32 log does not: on an
+    AVX-512 host it is off by up to 3 ulp for about 4 % of arguments, and the rain branch (Eq. 15) amplifies that far
+    beyond a float32 ulp of the code.  The float64 log rounded to float32 is the correctly rounded float32 log on
+    every host."""
     with np.errstate(all="ignore"):
-        log_d0 = np.log(np.asarray(d0, dtype=np.float32)).astype(np.float64)
+        log_d0 = np.log(np.asarray(d0, dtype=np.float32).astype(np.float64)).astype(np.float32).astype(np.float64)
     t, p, h, d0 = (np.asarray(v, dtype=np.float64) for v in (t, p, h, d0))
     dl = DAY_LENGTHS[lat_band, int(mth) - 1]
     with np.errstate(all="ignore"):

@@ -1,6 +1,8 @@
 """The DEVICE code of the fire-weather kernel (xclim_b200/csrc/fwi_core.cuh), compiled for the host, against
 the reference fixtures and the oracle.  The CUDA kernel adds only the thread-to-cell mapping to this code
 (xclim_b200/csrc/fwi.cu); its run on a GPU is tests/test_zzz_gpu_fire.py."""
+import os
+
 import numpy as np
 import pytest
 
@@ -90,60 +92,41 @@ def test_elementwise_functions_of_the_host_build(golden):  # noqa: F811
     assert hb.elementwise("BUI", np.zeros(1, np.float32), np.zeros(1, np.float32))[0] == 0
 
 
-@pytest.mark.skipif(not __import__("_ref_extract").available(), reason="reference sources not present (GPU box)")
-def test_every_mode_combination_against_the_live_reference():
+def check_against_stored_reference(golden_dir, group, exact_frac):
+    """The oracle and the host build of the device code on every case of `group` (tests/golden/make_golden.py)
+    against the outputs of the reference's `_fire_weather_calc` stored for it: every stored value within the
+    tolerances of check_outputs, and the bit-identical share of each code, over all cases, above `exact_frac`.
+    Returns the number of cases."""
+    g = np.load(os.path.join(golden_dir, "ref_cffwis_modes.npz"))
+    tc = lambda a: np.ascontiguousarray(a.T)   # noqa: E731
+    same = {}
+    n = 0
+    for i, (label, inp, state, mask, outs, over) in enumerate(mg.CFFWIS_CASE_GROUPS[group]()):
+        C, T = inp["tas"].shape
+        exp = mg.stored_cffwis_outputs(g, group, i, outs, C, T)
+        t, c = mg.sample_positions(C, T, i)
+        args = (tc(inp["tas"]), tc(inp["pr"]), tc(inp["hurs"]), tc(inp["ws"]), tc(inp["snd"]), inp["mth"], inp["lat"],
+                None if mask is None else tc(mask), *state)
+        for who, got in (("oracle", FO.fire_weather_calc(*args, outputs=outs, **over)),
+                         ("host build", hb.run(*args, outputs=outs, **over))):
+            got = {o: (np.asarray(v)[t, c] if o in mg.CFFWIS_FLOAT_OUTPUTS else np.asarray(v)) for o, v in got.items()}
+            check_outputs(got, exp, f"{who}:{label}", exact_frac=0.0)
+            for o in ("DC", "DMC", "FFMC", "winter_pr"):
+                if o in exp:
+                    k = same.setdefault((who, o), [0, 0])
+                    k[0] += int(((got[o] == exp[o]) | np.isnan(exp[o])).sum())
+                    k[1] += exp[o].size
+        n += 1
+    for (who, o), (k, m) in same.items():
+        assert k / m > exact_frac, f"{who}:{o}: {k} of {m} values bit-identical"
+    return n
+
+
+def test_every_mode_combination_against_the_reference(golden_dir):
     """All combinations of season method x overwintering x dry start x initial_start_up, each with random
     thresholds / window lengths / previous codes: the oracle AND the host build of the device code against the
-    reference's `_fire_weather_calc` executed where it lies."""
-    import itertools
-    import warnings
-
-    import _ref_extract as ref
-    fw = ref.load_cffwis()
-    rng = np.random.default_rng(123)
-    T = 320
-    combos = itertools.product([None, "mask", "WF93", "LA08", "GFWED"], [False, True], [None, "CFS", "GFWED", "GFWED+SNOW"],
-                               [True, False])
-    n = 0
-    for trial, (season, ow, dry, isu) in enumerate(combos):
-        if ow and season is None:
-            continue
-        inp = mg.cffwis_inputs(seed=1000 + trial, C=16, T=T)
-        dc0, dmc0, ffmc0, wpr = mg.cffwis_state(inp, [None, "some", "all"][trial % 3])
-        over = dict(season_method=season, overwintering=ow, dry_start=dry, initial_start_up=isu,
-                    temp_condition_days=int(rng.integers(1, 6)), snow_condition_days=int(rng.integers(1, 6)),
-                    snow_cover_days=int(rng.integers(5, 70)), temp_start_thresh=float(rng.uniform(8, 14)),
-                    temp_end_thresh=float(rng.uniform(2, 7)), snow_thresh=float(rng.choice([0.01, 0.03])),
-                    prec_thresh=float(rng.choice([1.0, 2.5])), dc_dry_factor=int(rng.integers(2, 7)),
-                    dmc_dry_factor=int(rng.integers(1, 4)), snow_min_cover_frac=float(rng.uniform(0.3, 0.8)),
-                    snow_min_mean_depth=float(rng.uniform(0.02, 0.1)), carry_over_fraction=float(rng.choice([0.5, 0.75, 1.0])),
-                    wetting_efficiency_fraction=float(rng.choice([0.5, 0.75, 0.9])))
-        outs = ["DC", "DMC", "FFMC", "ISI", "BUI", "FWI", "DSR"]
-        mask = None
-        if season == "mask":                      # a persistent random mask
-            mask = np.zeros((16, T), bool)
-            st = rng.random(16) < 0.5
-            for t in range(T):
-                st = np.where(rng.random(16) < 0.03, ~st, st)
-                mask[:, t] = st
-        elif season is not None:
-            outs.append("season_mask")
-        if ow:
-            outs.append("winter_pr")
-        kw = mg.cffwis_params(fw, outputs=outs, **over)
-        with warnings.catch_warnings():
-            warnings.simplefilter("ignore")
-            res = fw["_fire_weather_calc"](inp["tas"], inp["pr"], inp["hurs"], inp["ws"], inp["snd"], inp["mth"], inp["lat"],
-                                           mask, dc0.copy(), dmc0.copy(), ffmc0.copy(), wpr.copy(), **kw)
-        exp = {o: (np.asarray(a).T if np.asarray(a).ndim == 2 else np.asarray(a)) for o, a in zip(outs, res)}
-        tc = lambda a: np.ascontiguousarray(a.T)   # noqa: E731
-        args = (tc(inp["tas"]), tc(inp["pr"]), tc(inp["hurs"]), tc(inp["ws"]), tc(inp["snd"]), inp["mth"], inp["lat"],
-                None if mask is None else np.ascontiguousarray(mask.T), dc0, dmc0, ffmc0, wpr)
-        label = f"{season},{ow},{dry},{isu}"
-        check_outputs(FO.fire_weather_calc(*args, outputs=outs, **over), exp, "oracle:" + label, exact_frac=0.98)
-        check_outputs(hb.run(*args, outputs=outs, **over), exp, "host build:" + label, exact_frac=0.98)
-        n += 1
-    assert n == 72
+    reference's `_fire_weather_calc`."""
+    assert check_against_stored_reference(golden_dir, "modes", exact_frac=0.98) == 72
 
 
 def test_ring_mean_rounds_as_numpy_mean():
@@ -163,43 +146,9 @@ def test_ring_mean_rounds_as_numpy_mean():
             assert np.float32(got) == np.mean(vals), (n, head)
 
 
-@pytest.mark.skipif(not __import__("_ref_extract").available(), reason="reference sources not present (GPU box)")
-def test_branch_point_inputs_against_the_live_reference():
+def test_branch_point_inputs_against_the_reference(golden_dir):
     """Inputs drawn from the branch points of the equations (rain thresholds 0.5 / 1.5 / 2.8 mm and just above,
     humidity 0 and 100 %, calm and storm winds, temperatures at -2.8 / -1.1 / 21.1 degC, snow depth at its
     threshold, latitudes on the band edges, previous codes at 0 / 33 / 65 / 101), with and without missing
-    values: oracle and host build of the device code against the reference executed where it lies."""
-    import warnings
-
-    import _ref_extract as ref
-    fw = ref.load_cffwis()
-    rng = np.random.default_rng(7)
-    C, T = 32, 240
-    f32 = lambda a: np.ascontiguousarray(a, dtype=np.float32)   # noqa: E731
-    for trial in range(6):
-        tas = rng.choice([-45.0, -2.8, -1.1, 0.0, 21.1, 35.0, 50.0], size=(C, T)) + rng.normal(0, 0.5, (C, T))
-        pr = rng.choice([0.0, 0.5, 0.50001, 1.5, 1.50001, 2.8, 2.80001, 50.0, 300.0], size=(C, T))
-        hurs = rng.choice([0.0, 1e-3, 5.0, 50.0, 99.999, 100.0], size=(C, T))
-        ws = rng.choice([0.0, 1e-3, 10.0, 100.0, 250.0], size=(C, T))
-        snd = rng.choice([0.0, 0.01, 0.010001, 0.5], size=(C, T))
-        if trial % 3 == 0:
-            for a in (tas, pr, hurs, ws):
-                a[rng.random((C, T)) < 0.002] = np.nan
-        mth = rng.integers(1, 13, T).astype(np.int64)
-        lat = rng.choice([-90, -30, -15, 15, 30, 90, -29.999, 14.999, 0], size=C).astype(np.float64)
-        dc0, dmc0, ffmc0, wpr = mg.cffwis_state({"tas": f32(tas)}, [None, "some", "all"][trial % 3])
-        if trial % 3:
-            dc0[:4], dmc0[:4], ffmc0[:4] = [0.0, 1e-3, 800.0, 2000.0], [0.0, 33.0, 65.0, 500.0], [0.0, 101.0, 50.0, 99.9]
-        for season, ow, dry in ((None, False, None), ("WF93", True, "CFS"), ("GFWED", False, "GFWED+SNOW"), ("LA08", True, None)):
-            outs = ["DC", "DMC", "FFMC", "ISI", "BUI", "FWI", "DSR"] + (["season_mask"] if season else []) + \
-                (["winter_pr"] if ow else [])
-            over = dict(season_method=season, overwintering=ow, dry_start=dry, snow_cover_days=10)
-            kw = mg.cffwis_params(fw, outputs=outs, **over)
-            with warnings.catch_warnings():
-                warnings.simplefilter("ignore")
-                res = fw["_fire_weather_calc"](f32(tas), f32(pr), f32(hurs), f32(ws), f32(snd), mth, lat, None, dc0.copy(),
-                                               dmc0.copy(), ffmc0.copy(), wpr.copy(), **kw)
-            exp = {o: (np.asarray(a).T if np.asarray(a).ndim == 2 else np.asarray(a)) for o, a in zip(outs, res)}
-            args = tuple(f32(a.T) for a in (tas, pr, hurs, ws, snd)) + (mth, lat, None, dc0, dmc0, ffmc0, wpr)
-            check_outputs(FO.fire_weather_calc(*args, outputs=outs, **over), exp, f"oracle {trial} {season}", exact_frac=0.97)
-            check_outputs(hb.run(*args, outputs=outs, **over), exp, f"host build {trial} {season}", exact_frac=0.97)
+    values: oracle and host build of the device code against the reference's `_fire_weather_calc`."""
+    assert check_against_stored_reference(golden_dir, "branch", exact_frac=0.97) == 24

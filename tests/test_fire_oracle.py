@@ -1,7 +1,7 @@
 """The fire-weather oracle (oracle/fire_oracle.py) against the reference's own numba / numpy cores:
 fixtures made by executing indices/fire/_cffwis.py where it lies (tests/golden/make_golden.py), the
-reference tests' known answers (tests/test_cffwis.py:122-170), and a live cross-check where the reference
-sources are present."""
+reference tests' known answers (tests/test_cffwis.py:122-170), and the reference's step functions on a seeded
+sample of their arguments (tests/golden/make_golden.py)."""
 import os
 import sys
 
@@ -13,7 +13,6 @@ from oracle import fire_oracle as FO
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "golden"))
 import make_golden as mg  # noqa: E402
-import _ref_extract as ref  # noqa: E402
 
 
 @pytest.fixture(scope="module")
@@ -97,23 +96,16 @@ def test_reference_known_answers():
         FO.day_length_band(91)
 
 
-@pytest.mark.skipif(not ref.available(), reason="reference sources not present (GPU box)")
-def test_live_cross_check_of_the_step_functions():
-    fw = ref.load_cffwis()
-    rng = np.random.default_rng(3)
-    n = 4000
-    t = (rng.uniform(-15, 38, n)).astype(np.float32)
-    p = np.where(rng.random(n) < 0.5, 0, rng.gamma(0.8, 6, n)).astype(np.float32)
-    w = rng.uniform(0, 50, n).astype(np.float32)
-    h = rng.uniform(3, 100, n).astype(np.float32)
-    f0 = rng.uniform(0, 101, n).astype(np.float32)
-    d0 = rng.uniform(0, 200, n).astype(np.float32)
-    c0 = rng.uniform(0, 900, n).astype(np.float32)
-    for lat in (-50.0, -20.0, 0.0, 20.0, 50.0):
-        for mth in (1, 4, 7, 10):
-            band = FO.day_length_band(np.full(n, lat))
-            fb = FO.day_length_factor_band(np.full(n, lat))
-            np.testing.assert_allclose(FO.dmc_step(t, p, h, mth, band, d0), fw["_duff_moisture_code"](t, p, h, mth, lat, d0),
-                                       rtol=1e-6)     # the float32 log differs by an ulp between numpy and libm
-            np.testing.assert_allclose(FO.dc_step(t, p, mth, fb, c0), fw["_drought_code"](t, p, mth, lat, c0), rtol=1e-13)
-    np.testing.assert_allclose(FO.ffmc_step(t, p, w, h, f0), fw["_fine_fuel_moisture_code"](t, p, w, h, f0), rtol=1e-12)
+def test_step_functions_against_stored_reference_outputs(golden_dir):
+    g = np.load(os.path.join(golden_dir, "ref_cffwis_steps.npz"))
+    a, lats, mths = mg.cffwis_step_inputs()
+    for li, lat in enumerate(lats):
+        for mi, mth in enumerate(mths):
+            s = g["sel"][li, mi]
+            band = FO.day_length_band(np.full(s.size, lat))
+            fb = FO.day_length_factor_band(np.full(s.size, lat))
+            np.testing.assert_allclose(FO.dmc_step(a["t"][s], a["p"][s], a["h"][s], mth, band, a["d0"][s]), g["dmc"][li, mi],
+                                       rtol=1e-6)     # the C library's float32 log is not correctly rounded everywhere
+            np.testing.assert_allclose(FO.dc_step(a["t"][s], a["p"][s], mth, fb, a["c0"][s]), g["dc"][li, mi], rtol=1e-13)
+    s = g["sel_ffmc"]
+    np.testing.assert_allclose(FO.ffmc_step(a["t"][s], a["p"][s], a["w"][s], a["h"][s], a["f0"][s]), g["ffmc"], rtol=1e-12)

@@ -1,6 +1,6 @@
 """Pin the CPU oracle: (1) against fixtures produced by the reference's own numpy/numba cores
 (tests/golden/make_golden.py), (2) against the known-answer values held by the reference's tests,
-(3) live against the reference sources when /root/reference is present (authoring container)."""
+(3) against outputs of the reference's own cores on seeded inputs (tests/golden/make_golden.py)."""
 import os
 import sys
 
@@ -10,7 +10,7 @@ import pytest
 from oracle import xclim_oracle as O
 
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-import _ref_extract as ref  # noqa: E402
+import make_golden as mg  # noqa: E402
 
 
 # ------------------------------------------------------------------ fixtures from the reference
@@ -171,25 +171,14 @@ def test_spell_mask_truth_tables():
         np.testing.assert_array_equal(got, exp, err_msg=f"{win} {red} {op}")
 
 
-# ------------------------------------------------------------------ live cross-check (authoring container only)
-@pytest.mark.skipif(not ref.available(), reason="reference sources not present (GPU box)")
-def test_live_against_reference_sources():
-    rl = ref.load_run_length()
-    ut = ref.load_utils()
-    rng = np.random.default_rng(7)
-    m = rng.random((200, 50)) < 0.6
-    for red in ("max", "min", "sum", "count", "mean", "std"):
-        for w in (1, 2, 4):
-            got = O.rle_statistics(m, red, w)
-            exp = np.array([rl["statistics_run_1d"](m[:, i], red, w) for i in range(m.shape[1])], dtype=float)
-            np.testing.assert_allclose(got, exp, rtol=1e-12)
-    x = (rng.standard_normal((50, 150)) * 5 + 280).astype(np.float32)
-    x[rng.random(x.shape) < 0.05] = np.nan
-    import warnings
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        exp = ut["calc_perc"](x.copy(), [10.0, 90.0], 1 / 3, 1 / 3)
-    np.testing.assert_array_equal(O.calc_perc(x, [10.0, 90.0], 1 / 3, 1 / 3), exp)
+# ------------------------------------------------------------------ stored outputs of the reference's cores
+def test_against_stored_reference_outputs(golden_dir):
+    g = np.load(os.path.join(golden_dir, "ref_cross_check.npz"))
+    m, x = mg.cross_check_inputs()
+    for ri, red in enumerate(mg.CROSS_CHECK_REDUCERS):
+        for wi, w in enumerate(mg.CROSS_CHECK_WINDOWS):
+            np.testing.assert_allclose(O.rle_statistics(m, red, w), g["stats"][ri, wi], rtol=1e-12, err_msg=f"{red} w={w}")
+    np.testing.assert_array_equal(O.calc_perc(x, list(mg.CROSS_CHECK_PERCENTILES), 1 / 3, 1 / 3), g["calc_perc"])
 
 
 def _warm(d1, d2, n=365, start="2000-01-01"):

@@ -96,74 +96,25 @@ def test_fire_weather_streams_from_files_on_device(cuda, tmp_path):
 
 def test_kernel_every_mode_combination_against_the_oracle(cuda):
     """All season x overwintering x dry-start x initial_start_up combinations with random parameters: the kernel
-    against the oracle, which tests/test_fire_host_core.py pins to the live reference on the SAME combinations
+    against the oracle, which tests/test_fire_host_core.py pins to the reference on the SAME combinations
     (there, with the host build of this kernel's device code)."""
-    import itertools
-    rng = np.random.default_rng(123)
-    T = 320
-    n = 0
-    for trial, (season, ow, dry, isu) in enumerate(itertools.product(
-            [None, "mask", "WF93", "LA08", "GFWED"], [False, True], [None, "CFS", "GFWED", "GFWED+SNOW"], [True, False])):
-        if ow and season is None:
-            continue
-        inp = mg.cffwis_inputs(seed=1000 + trial, C=16, T=T)
-        dc0, dmc0, ffmc0, wpr = mg.cffwis_state(inp, [None, "some", "all"][trial % 3])
-        over = dict(season_method=season, overwintering=ow, dry_start=dry, initial_start_up=isu,
-                    temp_condition_days=int(rng.integers(1, 6)), snow_condition_days=int(rng.integers(1, 6)),
-                    snow_cover_days=int(rng.integers(5, 70)), temp_start_thresh=float(rng.uniform(8, 14)),
-                    temp_end_thresh=float(rng.uniform(2, 7)), snow_thresh=float(rng.choice([0.01, 0.03])),
-                    prec_thresh=float(rng.choice([1.0, 2.5])), dc_dry_factor=int(rng.integers(2, 7)),
-                    dmc_dry_factor=int(rng.integers(1, 4)), snow_min_cover_frac=float(rng.uniform(0.3, 0.8)),
-                    snow_min_mean_depth=float(rng.uniform(0.02, 0.1)), carry_over_fraction=float(rng.choice([0.5, 0.75, 1.0])),
-                    wetting_efficiency_fraction=float(rng.choice([0.5, 0.75, 0.9])))
-        outs = ["DC", "DMC", "FFMC", "ISI", "BUI", "FWI", "DSR"]
-        mask = None
-        if season == "mask":
-            m = np.zeros((16, T), bool)
-            st = rng.random(16) < 0.5
-            for t in range(T):
-                st = np.where(rng.random(16) < 0.03, ~st, st)
-                m[:, t] = st
-            mask = np.ascontiguousarray(m.T)
-        elif season is not None:
-            outs.append("season_mask")
-        if ow:
-            outs.append("winter_pr")
-        tc = lambda a: np.ascontiguousarray(a.T)   # noqa: E731
-        args = (tc(inp["tas"]), tc(inp["pr"]), tc(inp["hurs"]), tc(inp["ws"]), tc(inp["snd"]), inp["mth"], inp["lat"], mask,
-                dc0, dmc0, ffmc0, wpr)
-        exp = FO.fire_weather_calc(*args, outputs=outs, **over)
-        got = run_on_device(args, dict(outputs=outs, **over))
-        check_outputs(got, {k: np.asarray(v) for k, v in exp.items()}, f"{season},{ow},{dry},{isu}", exact_frac=0.90)
-        n += 1
-    assert n == 72
+    assert kernel_against_the_oracle(mg.cffwis_mode_cases()) == 72
 
 
 def test_kernel_branch_point_inputs_against_the_oracle(cuda):
-    """The branch-point inputs of tests/test_fire_host_core.py::test_branch_point_inputs_against_the_live_reference
+    """The branch-point inputs of tests/test_fire_host_core.py::test_branch_point_inputs_against_the_reference
     (there: oracle and host build against the reference), here the kernel against the oracle."""
-    rng = np.random.default_rng(7)
-    C, T = 32, 240
-    f32 = lambda a: np.ascontiguousarray(a, dtype=np.float32)   # noqa: E731
-    for trial in range(6):
-        tas = rng.choice([-45.0, -2.8, -1.1, 0.0, 21.1, 35.0, 50.0], size=(C, T)) + rng.normal(0, 0.5, (C, T))
-        pr = rng.choice([0.0, 0.5, 0.50001, 1.5, 1.50001, 2.8, 2.80001, 50.0, 300.0], size=(C, T))
-        hurs = rng.choice([0.0, 1e-3, 5.0, 50.0, 99.999, 100.0], size=(C, T))
-        ws = rng.choice([0.0, 1e-3, 10.0, 100.0, 250.0], size=(C, T))
-        snd = rng.choice([0.0, 0.01, 0.010001, 0.5], size=(C, T))
-        if trial % 3 == 0:
-            for a in (tas, pr, hurs, ws):
-                a[rng.random((C, T)) < 0.002] = np.nan
-        mth = rng.integers(1, 13, T).astype(np.int64)
-        lat = rng.choice([-90, -30, -15, 15, 30, 90, -29.999, 14.999, 0], size=C).astype(np.float64)
-        dc0, dmc0, ffmc0, wpr = mg.cffwis_state({"tas": f32(tas)}, [None, "some", "all"][trial % 3])
-        if trial % 3:
-            dc0[:4], dmc0[:4], ffmc0[:4] = [0.0, 1e-3, 800.0, 2000.0], [0.0, 33.0, 65.0, 500.0], [0.0, 101.0, 50.0, 99.9]
-        for season, ow, dry in ((None, False, None), ("WF93", True, "CFS"), ("GFWED", False, "GFWED+SNOW"), ("LA08", True, None)):
-            outs = ["DC", "DMC", "FFMC", "ISI", "BUI", "FWI", "DSR"] + (["season_mask"] if season else []) + \
-                (["winter_pr"] if ow else [])
-            over = dict(season_method=season, overwintering=ow, dry_start=dry, snow_cover_days=10)
-            args = tuple(f32(a.T) for a in (tas, pr, hurs, ws, snd)) + (mth, lat, None, dc0, dmc0, ffmc0, wpr)
-            exp = FO.fire_weather_calc(*args, outputs=outs, **over)
-            got = run_on_device(args, dict(outputs=outs, **over))
-            check_outputs(got, {k: np.asarray(v) for k, v in exp.items()}, f"{trial} {season}", exact_frac=0.90)
+    assert kernel_against_the_oracle(mg.cffwis_branch_cases()) == 24
+
+
+def kernel_against_the_oracle(cases):
+    tc = lambda a: np.ascontiguousarray(a.T)   # noqa: E731
+    n = 0
+    for label, inp, state, mask, outs, over in cases:
+        args = (tc(inp["tas"]), tc(inp["pr"]), tc(inp["hurs"]), tc(inp["ws"]), tc(inp["snd"]), inp["mth"], inp["lat"],
+                None if mask is None else tc(mask), *state)
+        exp = FO.fire_weather_calc(*args, outputs=outs, **over)
+        got = run_on_device(args, dict(outputs=outs, **over))
+        check_outputs(got, {k: np.asarray(v) for k, v in exp.items()}, label, exact_frac=0.90)
+        n += 1
+    return n
