@@ -465,7 +465,9 @@ __device__ __forceinline__ T pick_uniform(const T (&a)[N], int j) {
 // the batch, quarter grid, HBM time 1.75 ms): integer state, 4 cells per thread 19.1 ms (255 registers);
 // unit list + 2 cells 15.4 ms; float state 13.3 ms (ncu: ALU pipe 74 %, 18 FSEL + 18 ISETP per element in
 // the select chains, long_scoreboard 50 % at 16 warps per SM).
-// VEC / UNROLL: light passes (no run outputs) take 4 cells per thread, the others 2 cells and more rows in flight.
+// VEC / UNROLL: light passes (no run outputs) take 4 cells per thread, the others 2 cells and more rows in flight;
+// grids that cannot be read 16 bytes at a time (cell count or row stride not a multiple of 4, unaligned buffers) take
+// 1 cell per thread.
 template <int NC, int NCR, int NM, int NS, int VEC, int UNROLL>
 __global__ void __launch_bounds__(kThreads)
 period_multi_kernel(const float* __restrict__ x, int64_t C, int64_t ldx, const int32_t* __restrict__ poff,
@@ -603,7 +605,10 @@ int32_t launch_multi(const float* x, int64_t C, int64_t ldx, const int32_t* poff
                      float* out, cudaStream_t st) {
   // 4 cells per thread only pays for the lightest passes (measured: conditional sums are bound by the
   // float32 -> float64 conversions on the XU pipe, more conditions by registers)
-  if constexpr (NCR == 0 && NM == 0 && NS == 0 && NC <= 2) {
+  if (!can_vec4(x, C, ldx, out, nullptr)) {
+    period_multi_kernel<NC, NCR, NM, NS, 1, kUnroll><<<grid_for(C, 1, P), kThreads, 0, st>>>(x, C, ldx, poff, plan,
+                                                                                           out, (int64_t)P * C);
+  } else if constexpr (NCR == 0 && NM == 0 && NS == 0 && NC <= 2) {
     period_multi_kernel<NC, NCR, NM, NS, 4, 8><<<grid_for(C, 4, P), kThreads, 0, st>>>(x, C, ldx, poff, plan, out,
                                                                                         (int64_t)P * C);
   } else {
@@ -794,7 +799,6 @@ extern "C" int32_t xc_period_multi_f32(const float* x, int64_t T, int64_t C, int
              "plan holds at most %d conditions, %d run outputs (an even number), %d run sums and %d conditional sums",
              XC_MULTI_MAX_COND, XC_MULTI_MAX_RUNS, XC_MULTI_MAX_MSUM, XC_MULTI_MAX_SUMS);
   XC_REQUIRE(pl.n_runs / 2 <= pl.n_cond && (pl.n_msum == 0 || pl.n_cond > 0), "run outputs need their condition");
-  XC_REQUIRE(can_vec4(x, C, ldx, out, nullptr), "xc_period_multi_f32 needs C, ldx multiples of 4 and 16-byte aligned buffers");
   auto slot_ok = [&](int32_t sl) { return sl >= -1 && sl < n_slots; };
   bool ok = slot_ok(pl.slot_sum) && slot_ok(pl.slot_mean) && slot_ok(pl.slot_min) && slot_ok(pl.slot_max);
   // entries beyond the declared counts are neutralised (the rounded-up instantiation computes and drops them)

@@ -435,9 +435,12 @@ def period_run_quantile(x2d, poff, op_code, thr, q, window, resample_before_rl=T
 # ------------------------------------------------------------------------------------ fused multi-output pass
 def normalise_condition(op_code, thr):
     """(sgn, thr') with  x op thr  <=>  sgn * x > thr'  for every float32 x (NaN: False on both sides).
-    ``thr`` is compared in float32 (numpy >= 2 weak-scalar rule, indices/generic.py:301-326)."""
+    ``thr`` is compared in float32 (numpy >= 2 weak-scalar rule, indices/generic.py:301-326).
+    ``x >= -inf`` and ``x <= inf`` (true for every x but NaN) have no such form and are refused."""
     t = np.float32(thr)
     gt, lt, ge, le = _lib.OPS[">"], _lib.OPS["<"], _lib.OPS[">="], _lib.OPS["<="]
+    if (op_code == ge and t == -np.inf) or (op_code == le and t == np.inf):
+        raise NotImplementedError("the fused pass cannot express `x >= -inf` or `x <= inf`")
     if op_code == gt:
         return 1.0, float(t)
     if op_code == lt:

@@ -796,7 +796,7 @@ class _PassBuilder:
                     setattr(plan, "slot_" + st, slot(("stat", st)))
             # pick the places of this launch: run-owning places first (at most MAX_RUNS / 2), a max-sum owner at 0
             take, rest = [], []
-            n_run_places = 0
+            n_run_places = 0     # a max-sum owner without runs of its own counts: it holds run place 0 (ncr += 1 below)
             have_ms = False
             for pl in places:
                 owns_runs = bool(pl["runs"])
@@ -809,7 +809,7 @@ class _PassBuilder:
                     rest.append(pl)
                     continue
                 take.append(pl)
-                n_run_places += owns_runs
+                n_run_places += owns_runs or owns_ms
                 have_ms = have_ms or owns_ms
             # order: max-sum owner, then run owners, then the plain ones
             take.sort(key=lambda pl: (not (pl["first"] and pl["c"]["ms"] is not None), not pl["runs"]))
